@@ -46,7 +46,21 @@ def parse():
     ap.add_argument("--train-rays-per-warp", type=int, default=0)
     ap.add_argument("--render-warps", type=int, default=0, help="warps per CTA of the fused renderer (12)")
     ap.add_argument("--query-warps", type=int, default=0, help="warps per CTA of the point-query kernel (12 / 16 / 20)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step (rgb, depth, alpha, counter of rank 0) as DIR/<name>.npy, float32")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU frame (--impl ours)")
+    return args
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: one float32 DIR/<name>.npy per array, so that two builds can be compared output for output"""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "outputs above 64 MB: store a seeded sample instead"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -547,6 +561,9 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     device = torch.device("cuda", local)
+    # the occupancy-grid jitter of every frame is drawn inside the captured graph: seeded, the same arguments give the
+    # same frames from run to run
+    torch.manual_seed(0)
     if world > 1:
         dist.init_process_group("nccl", device_id=device)
     sampler = ClockSampler(local)
@@ -597,22 +614,25 @@ def run_ours(args):
             fn()
         barrier()
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+        out = None
         for a, b in ev:
             flush.zero_()  # L2 flush between timed iterations (outside the event bracket)
-            a.record(); fn(); b.record()
+            a.record(); out = fn(); b.record()
         barrier()
         ms = [a.elapsed_time(b) for a, b in ev]
         tot = torch.tensor([sum(ms)], device=device, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(tot, op=dist.ReduceOp.MAX)
-        return float(tot.item()), ms
+        return float(tot.item()), ms, out
 
     # nvidia-smi needs a few hundred ms before its first row: the sampler was started before the model was built
     t_load0 = time.monotonic()
     _lib.LAUNCHES = 0
-    total_ms, per = timed(step_resident, args.steps, max(args.warmup, 3))
+    total_ms, per, last = timed(step_resident, args.steps, max(args.warmup, 3))
     launches = getattr(_lib, "LAUNCHES", 0)
-    e2e_ms, _ = timed(step_e2e, args.steps, 3)
+    # the graph's output buffers are overwritten by every later replay: keep the last timed frame
+    last = dict(zip(("rgb", "depth", "alpha", "counter"), (t.clone() for t in last))) if args.dump_outputs else None
+    e2e_ms, _, _ = timed(step_e2e, args.steps, 3)
     t_load1 = time.monotonic()
     clocks = None
     if rank == 0:
@@ -683,6 +703,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if last is not None:
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in last.items()})
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

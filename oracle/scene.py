@@ -3,6 +3,7 @@ data: subject -> frame -> network -> occupancy grid -> rays.  Test infrastructur
 from __future__ import annotations
 
 import os
+import tempfile
 
 import numpy as np
 
@@ -11,7 +12,8 @@ from . import frame as oframe
 from . import render as orender
 
 f32 = np.float32
-_CACHE_DIR = os.environ.get("IA_ORACLE_CACHE", "/tmp/ia_oracle_cache")
+# per user: a cache directory another account created in the shared temporary directory would not be writable
+_CACHE_DIR = os.environ.get("IA_ORACLE_CACHE", os.path.join(tempfile.gettempdir(), f"ia_oracle_cache-{os.getuid()}"))
 
 
 def build_subject(resolution=128, track="male-3-casual", cache=True):

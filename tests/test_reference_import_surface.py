@@ -1,10 +1,12 @@
 """CPU: the reference's module paths resolve to the B200 mirror classes (SURVEY.md §8b).
 
-Every `_target_` string of /root/reference/confs/{renderer,deformer,network}/*.yaml and of the `model` / `loss` nodes of
+Every `_target_` string of the reference's confs/{renderer,deformer,network}/*.yaml and of the `model` / `loss` nodes of
 confs/SNARF_NGP*.yaml is resolved with importlib (no Hydra) through the `instant_avatar` alias package, the classes are
 checked to be the instantavatar_b200 ones, and the classes that construct without a GPU are instantiated from the
-reference's own YAML argument sets."""
+reference's own YAML argument sets.  What the reference's files hold is recorded in tests/golden/reference_conf.json
+(tests/golden/make_reference_conf_golden.py)."""
 import importlib
+import json
 import os
 
 import pytest
@@ -44,23 +46,22 @@ def test_target_resolves_to_the_mirror(conf, target, kwargs):
     assert cls is _resolve(MIRROR[target]), (target, cls)
 
 
-def test_targets_are_the_reference_files_targets():
-    """the committed list above equals what the reference's YAML files hold (only where /root/reference is mounted)"""
-    ref = "/root/reference"
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not mounted (GPU box)")
-    import re
-    found = set()
-    for sub in ("renderer", "deformer", "network"):
-        d = os.path.join(ref, "confs", sub)
-        for f in sorted(os.listdir(d)):
-            for m in re.finditer(r"_target_:\s*(\S+)", open(os.path.join(d, f)).read()):
-                found.add((f"confs/{sub}/{f}", m.group(1)))
+@pytest.fixture(scope="module")
+def reference_conf(golden_dir):
+    with open(os.path.join(golden_dir, "reference_conf.json")) as f:
+        return json.load(f)
+
+
+def test_targets_are_the_reference_files_targets(reference_conf):
+    """the committed list above equals what the reference's YAML files hold"""
+    found = {tuple(ct) for ct in reference_conf["conf_targets"]}
     committed = {(c, t) for c, t, _ in TARGETS if c.split("/")[1] in ("renderer", "deformer", "network")}
     assert found == committed, found ^ committed
-    for f in ("SNARF_NGP.yaml", "SNARF_NGP_refine.yaml", "SNARF_NGP_fitting.yaml", "demo.yaml"):
-        for m in re.finditer(r"_target_:\s*(\S+)", open(os.path.join(ref, "confs", f)).read()):
-            assert m.group(1) in MIRROR, (f, m.group(1))
+    assert set(reference_conf["top_level_targets"]) == {"SNARF_NGP.yaml", "SNARF_NGP_refine.yaml", "SNARF_NGP_fitting.yaml", "demo.yaml"}
+    for f, targets in reference_conf["top_level_targets"].items():
+        assert targets, f
+        for t in targets:
+            assert t in MIRROR, (f, t)
 
 
 def test_instantiate_cpu_constructible_targets():
@@ -96,22 +97,17 @@ def test_reference_import_statements():
     assert DensityGrid.__module__.startswith("instantavatar_b200") and SMPLParamEmbedding.__module__.startswith("instantavatar_b200")
 
 
-def test_reference_ngp_file_runs_on_the_tinycudann_shim():
-    """the reference's OWN models/networks/ngp.py, loaded from /root/reference by path, builds on the in-repo `tinycudann`
-    module: same sub-module names and flat parameter sizes (CPU: construction only; the forward is a GPU test)"""
-    import importlib.util
-    import sys
-    ref = "/root/reference/instant_avatar/models/networks/ngp.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not mounted (GPU box)")
-    import tinycudann  # the shim must win the import inside the reference file
+def test_reference_ngp_file_runs_on_the_tinycudann_shim(reference_conf):
+    """the tinycudann modules the reference's OWN models/networks/ngp.py builds (class and keyword arguments recorded from
+    that file) construct on the in-repo `tinycudann` module: same sub-module names and flat parameter sizes (CPU:
+    construction only; the forward is a GPU test)"""
+    import torch
+    import tinycudann
     assert "ia_b200" in tinycudann.__version__
-    spec = importlib.util.spec_from_file_location("_ref_ngp_under_shim", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    from instantavatar_b200.config import Cfg
-    net = mod.NeRFNGPNet(Cfg({"center": [0, -0.3, 0], "scale": [2.5, 2.5, 2.5]}))
+    ngp = reference_conf["ngp"]
+    net = torch.nn.Module()
+    for m in ngp["modules"]:
+        setattr(net, m["attr"], getattr(tinycudann, m["class"])(**m["kwargs"]))
     sizes = {k: v.numel() for k, v in net.named_parameters()}
-    assert sizes == {"encoder.params": 3072 + 2 * 6513496, "color_net.params": 6144}
-    assert set(dict(net.named_buffers())) == {"center", "scale"}
-    sys.modules.pop("_ref_ngp_under_shim", None)
+    assert sizes == ngp["parameters"] == {"encoder.params": 3072 + 2 * 6513496, "color_net.params": 6144}
+    assert ngp["buffers"] == ["center", "scale"]
